@@ -2,6 +2,7 @@
 """bench.py — rays/sec of the Mip-NeRF per-ray hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--precision bf16|fp16|fp32] [--impl reference]
+                    [--dump-outputs DIR]
 
 One "step" = one MipNerf.forward-equivalent (both levels, full 5-tuple written) over one batch of
 4096 synthetic Blender-shape rays at 128+128 samples (BASELINE configs[1]) on every rank; weights are
@@ -98,31 +99,14 @@ class ClockSampler:
 
 
 def _cpu_arm_setup():
-    """The CPU arm: the UNMODIFIED reference imported from baseline/_ref (tools/install_ref.py) when it is
-    installed (`kind` "reference"), else the oracle port (`kind` "port").  Returns (kind, forward) with
-    forward(state_dict, rays_tuple) -> list of per-level tuples, fp32, no_grad, randomized=False, white_bkgd=True."""
-    import torch
-    import mipnerf_pl_b200 as mp
-    try:
-        from baseline import ref_loader
-        RefMipNerf, RefRays, _ = ref_loader.load()
-        models = {}
+    """The CPU arm: the oracle port of the reference's forward, which reproduces the reference's outputs bit for bit
+    (tests/test_reference_arm.py).  Returns (kind, forward) with forward(state_dict, rays_tuple) -> list of per-level
+    tuples, fp32, no_grad, randomized=False, white_bkgd=True."""
+    from oracle import mipnerf_oracle as oracle  # allowed here: this IS the CPU arm
 
-        def forward(sd, rays):
-            m = models.get(id(sd))
-            if m is None:
-                m = RefMipNerf()                      # models/mip_nerf.py:117-141 defaults == BASELINE configs[1]
-                m.load_state_dict(sd)
-                models[id(sd)] = m.eval()
-            with torch.no_grad():
-                return m(RefRays(*rays), False, True)
-        return "reference", forward
-    except ImportError:
-        from oracle import mipnerf_oracle as oracle  # allowed here: this IS the CPU arm
-
-        def forward(sd, rays):
-            return oracle.forward(sd, oracle.Rays(*rays), False, True)
-        return "port", forward
+    def forward(sd, rays):
+        return oracle.forward(sd, oracle.Rays(*rays), False, True)
+    return "port", forward
 
 
 def pick_cpu_threads(forward):
@@ -165,8 +149,7 @@ def cpu_arm(forward, num_rays, steps, warmup):
     return num_rays / dt, dt, torch.get_num_threads()
 
 
-CPU_ARM_WHAT = {"reference": "the unmodified reference MipNerf.forward (models/mip_nerf.py:172-248) imported from baseline/_ref",
-                "port": "fp32 torch-CPU oracle (port of models/mip_nerf.py:172-248; baseline/_ref not installed)"}
+CPU_ARM_WHAT = {"port": "fp32 torch-CPU oracle (port of models/mip_nerf.py:172-248)"}
 
 
 def run_reference(args):
@@ -175,10 +158,9 @@ def run_reference(args):
         return
     kind, forward = _cpu_arm_setup()
     threads, rate = pick_cpu_threads(forward)
-    steps = max(1, args.steps)
     # bounded sample per step: the whole K-step run should take ~90 s of CPU time on this box
-    sample = int(min(BATCH, max(64, rate * 90.0 / steps)))
-    rps, dt, cores = cpu_arm(forward, sample, steps, max(1, min(args.warmup, 2)))
+    sample = int(min(BATCH, max(64, rate * 90.0 / args.steps)))
+    rps, dt, cores = cpu_arm(forward, sample, args.steps, max(1, min(args.warmup, 2)))
     line = {
         "impl": "reference", "metric": "rays/sec (4096-ray batch, 128+128 samples)", "value": rps,
         "unit": "rays/s", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
@@ -205,7 +187,7 @@ DTYPE = {"bf16": "bf16", "fp16": "f16", "fp32": "f32", "fp16x3": "f16x3 (split f
 
 def measure_parity(mp, model, dev):
     """Measured in this run: fine-level RGB of `model`'s precision against the fp32 CPU forward of the reference
-    (baseline/_ref, else the oracle port) on 256 rays, xavier and trained-like weights.  The checker only."""
+    (the oracle port) on 256 rays, xavier and trained-like weights.  The checker only."""
     import torch
     kind, forward = _cpu_arm_setup()
     out = {"checker": kind, "rays": 256, "floor": 0.02, "precision": model.precision}
@@ -227,6 +209,28 @@ def measure_parity(mp, model, dev):
     return out
 
 
+DUMP_MAX_BYTES = 63 << 20                # array data of --dump-outputs: under 64 MiB with the .npy headers
+
+
+def dump_outputs(out_dir, levels):
+    """What a caller of the timed forward receives: per level comp_rgb [B,3], distance [B], acc [B], weights [B,N] and
+    t_samples [B,N+1], written as <out_dir>/level<l>_<name>.npy in float32 (8.6 MB at the default 4096-ray batch).
+    A batch whose outputs exceed DUMP_MAX_BYTES is cut to a fixed sample of rays (seed 0, ascending ray order), the
+    same rays in every file."""
+    import numpy as np
+    names = ("comp_rgb", "distance", "acc", "weights", "t_samples")
+    arrays = {f"level{lvl}_{name}": t.detach().float().cpu().numpy()
+              for lvl, outs in enumerate(levels) for name, t in zip(names, outs)}
+    b = next(iter(arrays.values())).shape[0]
+    bytes_per_ray = sum(a.nbytes for a in arrays.values()) // max(b, 1)
+    if b * bytes_per_ray > DUMP_MAX_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(b, DUMP_MAX_BYTES // bytes_per_ray, replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -244,7 +248,11 @@ def main():
     ap.add_argument("--no-parity-mode", action="store_true",
                     help="skip the secondary measurement of the 1e-4 contract mode (fp16x3) in a bf16 / fp16 run (N = 1)")
     ap.add_argument("--no-parity", action="store_true", help="skip the in-run parity measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (rank 0) as DIR/<name>.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
@@ -310,7 +318,7 @@ def main():
 
         def timed(self, steps, fn=None):
             """K steps, device-timed with events on the launch stream, L2 flushed (untimed) between steps;
-            returns ms per step, max over ranks."""
+            returns ms per step, max over ranks.  `self.last` keeps what the last step returned."""
             fn = fn or self.step
             starts = [torch.cuda.Event(enable_timing=True) for _ in range(steps)]
             stops = [torch.cuda.Event(enable_timing=True) for _ in range(steps)]
@@ -318,7 +326,7 @@ def main():
             for i in range(steps):
                 flush.zero_()
                 starts[i].record()
-                fn()
+                self.last = fn()
                 stops[i].record()
             barrier()
             total = torch.tensor([sum(a.elapsed_time(b) for a, b in zip(starts, stops))], device=dev,
@@ -369,6 +377,8 @@ def main():
     wall = time.perf_counter() - wall0
     clocks = sampler.stop() if rank == 0 else None
     value = b_global / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, arm.last)
 
     # ---- instrumented pass: the same K steps launched eagerly with the library's CUDA-event bracket around every
     #      kernel launch (a graph replay cannot be bracketed per kernel): kernel list, launch counts, launch time

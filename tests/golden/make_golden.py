@@ -360,7 +360,16 @@ def density_noise_case():
                  white_bkgd=True, density_noise=1.0)
 
 
+def reference_arm_case():
+    # what bench.py's CPU arm computes: 96 rays of the benchmark's ray generator (seed 0), both weight sets
+    for kind in ("xavier", "trained_like"):
+        forward_case(f"reference_arm_{kind}.npz", 96, seed=0, weights_kind=kind, randomized=False, white_bkgd=True)
+
+
 if __name__ == "__main__":
+    if len(sys.argv) > 1 and sys.argv[1] == "reference_arm":   # regenerate only reference_arm_*.npz
+        reference_arm_case()
+        sys.exit(0)
     if len(sys.argv) > 1 and sys.argv[1] == "metrics":    # regenerate only metrics.npz
         metrics_case()
         sys.exit(0)
@@ -385,6 +394,7 @@ if __name__ == "__main__":
                  num_samples=64, num_levels=1)
     density_noise_case()
     degrees_case()
+    reference_arm_case()
     resampler_case()
     stages_case()
     training_case()

@@ -360,16 +360,19 @@ def test_ray_staging_single_copy_round_trip():
         assert torch.equal(a.pixels[lvl, 900:1200], a[lvl][1]) and torch.equal(a.pixels[lvl, 1200:], a[lvl][2])
 
 
-def test_bench_line_contract():
+def test_bench_line_contract(tmp_path):
     """bench.py on the GPU prints ONE JSON line with the keys the driver reads (value, e2e, roofline, clocks,
-    gpu_launches ...), a tensor-bound roofline for the fused level kernel and non-zero launch counts."""
+    gpu_launches ...), a tensor-bound roofline for the fused level kernel and non-zero launch counts.  With
+    --dump-outputs it writes what its last timed step computed: the forward's outputs on the bench's rays."""
     import json
     import os
     import subprocess
     import sys
     root = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
+    dump = tmp_path / "outputs"
     out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "5", "--warmup", "3",
-                          "--no-cpu-baseline", "--no-frame"], capture_output=True, text=True, timeout=600, cwd=root)
+                          "--no-cpu-baseline", "--no-frame", "--dump-outputs", str(dump)],
+                         capture_output=True, text=True, timeout=600, cwd=root)
     assert out.returncode == 0, out.stderr[-2000:]
     lines = [l for l in out.stdout.strip().splitlines() if l.startswith("{")]
     assert len(lines) == 1
@@ -385,3 +388,12 @@ def test_bench_line_contract():
     assert r["bound"] == "tensor" and r["kernel"] == "mlp_level_tc" and 0.2 < r["frac"] < 1.0
     assert abs(r["frac"] - r["achieved"] / r["peak"]) < 1e-9
     assert "workload" in d["config"]
+    model = mp.MipNerf(precision="bf16")
+    model.load_state_dict(make_state_dict(seed=0, kind="xavier"))
+    model = model.to("cuda").eval()
+    want = model(mp.namedtuple_map(lambda t: t.to("cuda"), mp.random_ray_batch(4096, seed=0)), False, True)
+    assert len(os.listdir(dump)) == 10
+    for lvl in range(2):
+        for k, name in enumerate(("comp_rgb", "distance", "acc", "weights", "t_samples")):
+            got = np.load(dump / f"level{lvl}_{name}.npy")
+            assert got.dtype == np.float32 and np.array_equal(got, want[lvl][k].cpu().numpy()), (lvl, name)

@@ -168,8 +168,7 @@ def test_bench_reference_arm_prints_contract_json():
                 "scaling", "vs_baseline", "dtype", "data", "config", "cpu_baseline", "e2e"):
         assert key in line, key
     assert line["impl"] == "reference" and line["unit"] == "rays/s" and line["value"] > 0
-    have_ref = os.path.exists(os.path.join(ROOT, "baseline", "_ref", "models", "mip_nerf.py"))
-    assert line["cpu_baseline"]["kind"] == ("reference" if have_ref else "port")
+    assert line["cpu_baseline"]["kind"] == "port"
     assert line["e2e"]["h2d_bytes_per_step"] == 0
 
 

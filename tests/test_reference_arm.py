@@ -1,87 +1,38 @@
-"""The CPU arm of bench.py is the UNMODIFIED reference when baseline/_ref is installed (tools/install_ref.py).
-Here: (1) the installed files are byte-identical to the manifest they were copied with, (2) the oracle port equals
-the reference bit for bit on the bench workload's rays and weights — so a box that only has the port (kind "port")
-times the same arithmetic."""
-import hashlib
-import json
+"""The CPU arm of bench.py computes what the UNMODIFIED reference computes.  The reference's own outputs on the bench
+workload's rays (seed 0) and weights are stored in tests/golden/reference_arm_{xavier,trained_like}.npz
+(tests/golden/make_golden.py); the oracle port, which bench.py times on the host, must reproduce them bit for bit."""
+import importlib.util
 import os
 
 import pytest
 import torch
 
-from helpers import ROOT, make_state_dict, oracle
+from helpers import ROOT, golden, golden_levels, golden_rays, make_state_dict, oracle
 
-import mipnerf_pl_b200 as mp
-
-ref_loader = pytest.importorskip("baseline.ref_loader")
-pytestmark = pytest.mark.skipif(not ref_loader.available(), reason="baseline/_ref not installed on this box")
+FIELDS = ("comp_rgb", "distance", "acc", "weights", "t_samples")
 
 
-def test_installed_reference_matches_manifest():
-    with open(os.path.join(ref_loader.REF_DIR, "MANIFEST.json")) as f:
-        man = json.load(f)
-    assert set(man["files"]) >= {"models/mip.py", "models/mip_nerf.py", "datasets/datasets.py"}
-    for rel, digest in man["files"].items():
-        with open(os.path.join(ref_loader.REF_DIR, rel), "rb") as f:
-            assert hashlib.sha256(f.read()).hexdigest() == digest, rel
-    src = man["source"]
-    if os.path.isdir(src):   # build container: still identical to the upstream tree
-        for rel in man["files"]:
-            with open(os.path.join(src, rel), "rb") as a, open(os.path.join(ref_loader.REF_DIR, rel), "rb") as b:
-                assert a.read() == b.read(), rel
+def assert_equals_reference(got, g, what):
+    want = golden_levels(g)
+    assert len(got) == len(want) == 2
+    for lvl in range(2):
+        for k, name in enumerate(FIELDS):
+            assert torch.equal(got[lvl][k], torch.from_numpy(want[lvl][k])), (what, lvl, name)
 
 
 @pytest.mark.parametrize("kind", ["xavier", "trained_like"])
 def test_port_equals_reference_bit_for_bit(kind):
-    RefMipNerf, RefRays, _ = ref_loader.load()
-    rays = mp.random_ray_batch(96, seed=0)
+    g = golden(f"reference_arm_{kind}.npz")
     sd = make_state_dict(seed=0, kind=kind)
-    model = RefMipNerf()
-    model.load_state_dict(sd)
-    with torch.no_grad():
-        want = model.eval()(RefRays(*rays), False, True)
-    got = oracle.forward(sd, oracle.Rays(*rays), False, True)
-    for lvl in range(2):
-        for k, name in enumerate(("comp_rgb", "distance", "acc", "weights", "t_samples")):
-            assert torch.equal(got[lvl][k], want[lvl][k]), (kind, lvl, name)
+    got = oracle.forward(sd, oracle.Rays(*golden_rays(g)), False, True)
+    assert_equals_reference(got, g, kind)
 
 
-def test_bench_cpu_arm_prefers_the_reference():
-    import importlib.util
+def test_bench_cpu_arm_computes_the_references_outputs():
     spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
     bench = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(bench)
     kind, forward = bench._cpu_arm_setup()
-    assert kind == "reference"
-    out = forward(make_state_dict(seed=0), mp.random_ray_batch(8, seed=0))
-    assert len(out) == 2 and out[1][0].shape == (8, 3)
-
-
-@pytest.mark.parametrize("name,kind,kw,shape", [
-    ("forward_density_noise.npz", "trained_like", dict(density_noise=1.0), {}),
-    ("forward_deg10_view2.npz", "trained_like", dict(max_deg_point=10, deg_view=2), dict(xyz_dim=60, view_dim=15)),
-])
-def test_round2_goldens_are_the_installed_references_outputs(name, kind, kw, shape):
-    """The fixtures added in round 2 (density noise, lower encoding degrees) re-derived from the unmodified reference in
-    baseline/_ref (bit for bit on the host that wrote them; the contract's 1e-4 elsewhere) — including the order in which the reference consumes its generator when density_noise >
-    0 (rand, randn, uniform_, randn; tests/golden/make_golden.py seeds it with 1234 + seed)."""
-    from helpers import golden, golden_levels, golden_rays
-    RefMipNerf, RefRays, _ = ref_loader.load()
-    g = golden(name)
-    seed, randomized, white = (int(v) for v in g["meta"])
-    model = RefMipNerf(**kw)
-    model.load_state_dict(make_state_dict(seed=seed, kind=kind, **shape))
-    rays = golden_rays(g)
-    torch.manual_seed(1234 + seed)
-    with torch.no_grad():
-        ret = model.eval()(RefRays(*rays), bool(randomized), bool(white))
-    from helpers import assert_level_close
-    exact = True
-    for lvl, want in enumerate(golden_levels(g)):
-        # the contract's tolerance everywhere (torch's sgemm may block differently on a host with another core count /
-        # ISA than the one that wrote the fixture) ...
-        assert_level_close(ret[lvl], want, what=f"{name} level {lvl} ", level=lvl)
-        exact = exact and all(torch.equal(ret[lvl][k], torch.from_numpy(want[k])) for k in range(5))
-    # ... the coarse fenceposts have no MLP upstream: bit-exact on any host
-    assert torch.equal(ret[0][4], torch.from_numpy(golden_levels(g)[0][4]))
-    print(f"{name}: {'bit-identical to' if exact else 'within 1e-4 of'} the committed fixture on this host")
+    assert kind == "port"
+    g = golden("reference_arm_xavier.npz")
+    assert_equals_reference(forward(make_state_dict(seed=0), golden_rays(g)), g, "bench CPU arm")
