@@ -199,6 +199,14 @@ int mipnerf_b200_forward_backward_rng(const mipnerf_b200_config* cfg, const mipn
                                       int precision, const mipnerf_b200_loss* loss, mipnerf_b200_level_out* outs,
                                       const mipnerf_b200_linear_grad* grads, int num_grads, int accumulate,
                                       void* workspace, size_t workspace_bytes, void* stream);
+/* The same with (seed, offset) read from DEVICE memory (`rng_state` = uint64_t[2]) when the kernels run, so that a
+ * CUDA graph that captured this call draws fresh numbers after the caller advances rng_state[1]: the draws equal
+ * forward_backward_rng's for the same values.  BF16 / FP16 fused step only (EUNSUPPORTED otherwise). */
+int mipnerf_b200_forward_backward_rng_state(const mipnerf_b200_config* cfg, const mipnerf_b200_weights* weights,
+                                            const mipnerf_b200_rays* rays, const uint64_t* rng_state, int white_bkgd,
+                                            int precision, const mipnerf_b200_loss* loss, mipnerf_b200_level_out* outs,
+                                            const mipnerf_b200_linear_grad* grads, int num_grads, int accumulate,
+                                            void* workspace, size_t workspace_bytes, void* stream);
 
 /* Stand-alone tensor-core linear layer  y[m,n] = act(x[m,k] . weight[n,k]^T + bias)  (tcgen05, 16-bit operands, fp32
  * accumulate; n in {128,256}, k in {96,128,256}): the GEMM the training step uses for its forward and dgrad passes in
@@ -226,6 +234,18 @@ int mipnerf_b200_adam_step(float* param, const float* grad, float* exp_avg, floa
 int mipnerf_b200_adam_step_multi(int count, float* const* params, const float* const* grads, float* const* exp_avg,
                                  float* const* exp_avg_sq, const int64_t* sizes, double lr, double beta1, double beta2,
                                  double eps, int64_t step, double grad_scale, void* stream);
+/* adam_step_multi with the step count on the device: the update number is t = *step + 1 and the step size lr_t / bc1_t
+ * and sqrt(bc2_t) are read from the DEVICE tables step_size[t] / bc2_sqrt[t] (t clamped to 1 .. table_len - 1), which
+ * the caller fills with the double-precision math of adam_step_multi; *step is not changed. */
+int mipnerf_b200_adam_step_multi_table(int count, float* const* params, const float* const* grads,
+                                       float* const* exp_avg, float* const* exp_avg_sq, const int64_t* sizes,
+                                       const float* step_size, const float* bc2_sqrt, int64_t table_len,
+                                       const int64_t* step, double beta1, double beta2, double eps, double grad_scale,
+                                       void* stream);
+/* End of a device-driven training step: ring[(*step % ring_len) * 2 + {0, 1}] = {*loss, *psnr} (ring_len may be 0),
+ * then *step += 1 and rng_state[1] += 1.  All pointers are device pointers. */
+int mipnerf_b200_train_step_advance(int64_t* step, uint64_t* rng_state, const float* loss, const float* psnr,
+                                    float* ring, int ring_len, void* stream);
 
 /* Pinhole rays of rows [row0,row0+rows) of an H x W frame generated on the device, replacing the
  * host NumPy loaders (datasets/datasets.py:214-263, render_video.py:29-105).  `c2w_host` is a HOST
@@ -254,6 +274,16 @@ int mipnerf_b200_rays_from_pixels(const float* cam_table, const int64_t* offsets
                                   int num_images, const int64_t* pixel_ids, int64_t count, const float* atlas,
                                   float* origins, float* directions, float* viewdirs, float* radii,
                                   float* lossmult, float* near_out, float* far_out, float* rgb, void* stream);
+/* A uniformly random batch of `count` training rays drawn on the device, then rays_from_pixels on it: the id of ray i is
+ * floor(x * num_pixels / 2^32), x the first 32-bit output of Philox4x32-10 keyed like the in-kernel draws by
+ * rng_state = DEVICE uint64_t[2] (seed, offset) with counter (ray_base + i, stream 64, offset).  1 <= num_pixels <= 2^32;
+ * each id's probability is within 2^-32 of 1/num_pixels.  Ids past offsets[num_images] (num_pixels larger than the
+ * atlas) are clamped to its last row.  pixel_ids [count] (nullable) receives the ids. */
+int mipnerf_b200_sample_pixels(const float* cam_table, const int64_t* offsets, const int32_t* widths, int num_images,
+                               int64_t num_pixels, const uint64_t* rng_state, int64_t ray_base, int64_t count,
+                               const float* atlas, int64_t* pixel_ids, float* origins, float* directions,
+                               float* viewdirs, float* radii, float* lossmult, float* near_out, float* far_out,
+                               float* rgb, void* stream);
 
 /* ---- per-stage entry points (unit parity against the functions of models/mip.py) ---- */
 

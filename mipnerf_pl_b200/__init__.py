@@ -13,9 +13,9 @@ from .ops import (sample_along_rays, resample_along_rays, cast_rays, integrated_
 from .weights import make_state_dict
 from .train import FusedAdam, MipLRDecay, allreduce_grads, forward_backward, fused_loss, mip_lr
 from .datasets import (Blender, Multicam, DeviceRayBank, Scene, dataset_dict, load_blender_scene, load_multicam_scene,
-                       image_rays, convert_blender_to_multiscale, write_synthetic_blender_scene)
+                       image_rays, convert_blender_to_multiscale, write_synthetic_blender_scene, philox_pixel_ids)
 from .render import generate_rays, render_frame, render_sharded, shard_bounds, shard_rows, gather_rows
-from .graph import GraphedForward
+from .graph import GraphedForward, GraphedTrainStep
 from .metrics import eval_errors, ssim, evaluate, render_path, spheric_path, save_images
 
 __all__ = [
@@ -26,6 +26,6 @@ __all__ = [
     "render_sharded", "shard_bounds", "shard_rows", "gather_rows", "FusedAdam", "MipLRDecay", "allreduce_grads",
     "forward_backward", "fused_loss", "mip_lr", "Blender", "Multicam", "DeviceRayBank", "Scene", "dataset_dict",
     "load_blender_scene", "load_multicam_scene", "image_rays", "convert_blender_to_multiscale",
-    "write_synthetic_blender_scene", "GraphedForward", "philox_uniform", "philox_normal", "eval_errors", "ssim", "evaluate",
+    "write_synthetic_blender_scene", "GraphedForward", "GraphedTrainStep", "philox_pixel_ids", "philox_uniform", "philox_normal", "eval_errors", "ssim", "evaluate",
     "render_path", "spheric_path", "save_images",
 ]

@@ -92,6 +92,9 @@ _SIGNATURES = {
     "mipnerf_b200_forward_backward_rng": (C.c_int, [C.POINTER(Config), C.POINTER(Weights), C.POINTER(RaysStruct),
                                                     C.POINTER(Rng), C.c_int, C.c_int, C.POINTER(Loss), C.POINTER(LevelOut),
                                                     C.POINTER(LinearGrad), C.c_int, C.c_int, _V, C.c_size_t, _V]),
+    "mipnerf_b200_forward_backward_rng_state": (C.c_int, [C.POINTER(Config), C.POINTER(Weights), C.POINTER(RaysStruct),
+                                                          _V, C.c_int, C.c_int, C.POINTER(Loss), C.POINTER(LevelOut),
+                                                          C.POINTER(LinearGrad), C.c_int, C.c_int, _V, C.c_size_t, _V]),
     "mipnerf_b200_linear_tc": (C.c_int, [_V, _V, _V, _V, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int, _V, C.c_size_t, _V]),
     "mipnerf_b200_wgrad_tc_scratch_bytes": (C.c_size_t, [C.c_int, C.c_int]),
     "mipnerf_b200_wgrad_tc": (C.c_int, [_V, C.c_int, _V, C.c_int, _V, C.c_int, C.c_int, C.c_int64, _V, _V, C.c_int, _V,
@@ -100,11 +103,16 @@ _SIGNATURES = {
                                          C.c_int64, C.c_double, _V]),
     "mipnerf_b200_adam_step_multi": (C.c_int, [C.c_int, _V, _V, _V, _V, _V, C.c_double, C.c_double, C.c_double,
                                                C.c_double, C.c_int64, C.c_double, _V]),
+    "mipnerf_b200_adam_step_multi_table": (C.c_int, [C.c_int, _V, _V, _V, _V, _V, _V, _V, C.c_int64, _V, C.c_double,
+                                                     C.c_double, C.c_double, C.c_double, _V]),
+    "mipnerf_b200_train_step_advance": (C.c_int, [_V, _V, _V, _V, _V, C.c_int, _V]),
     "mipnerf_b200_generate_rays": (C.c_int, [_f32p, C.c_int, C.c_int, C.c_float, C.c_float, C.c_float, C.c_int, C.c_int,
                                              _V, _V, _V, _V, _V, _V, _V]),
     "mipnerf_b200_image_metrics_scratch_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
     "mipnerf_b200_image_metrics": (C.c_int, [_V, _V, C.c_int, C.c_int, C.c_int, _V, C.c_size_t, _V, _V]),
     "mipnerf_b200_rays_from_pixels": (C.c_int, [_V, _V, _V, C.c_int, _V, C.c_int64, _V, _V, _V, _V, _V, _V, _V, _V, _V, _V]),
+    "mipnerf_b200_sample_pixels": (C.c_int, [_V, _V, _V, C.c_int, C.c_int64, _V, C.c_int64, C.c_int64, _V, _V, _V, _V,
+                                             _V, _V, _V, _V, _V, _V, _V]),
     "mipnerf_b200_sample_along_rays": (C.c_int, [C.POINTER(RaysStruct), C.c_int, C.c_int, C.c_int, _V, _V, _V, _V, _V]),
     "mipnerf_b200_cast_rays": (C.c_int, [C.POINTER(RaysStruct), _V, C.c_int, _V, _V, _V]),
     "mipnerf_b200_integrated_pos_enc": (C.c_int, [_V, _V, C.c_int64, C.c_int, C.c_int, _V, _V]),

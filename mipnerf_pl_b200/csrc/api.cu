@@ -519,7 +519,7 @@ static int forward_backward_fused(const mipnerf_b200_config* cfg, const Dims& d,
                                   const float* u_jitter, const mipnerf_b200_rng* rng, int white_bkgd, int precision,
                                   const mipnerf_b200_loss* loss, mipnerf_b200_level_out* outs,
                                   const mipnerf_b200_linear_grad* grads, bool* touched, void* workspace,
-                                  cudaStream_t st) {
+                                  cudaStream_t st, const uint64_t* rng_state) {
   const int n = cfg->num_samples, depth = cfg->net_depth, W = cfg->net_width, Wc = cfg->net_width_condition;
   const float rgb_scale = (float)(1.0 + 2.0 * (double)cfg->rgb_padding);
   const int64_t B = rays->num_rays;
@@ -566,6 +566,7 @@ static int forward_backward_fused(const mipnerf_b200_config* cfg, const Dims& d,
       lo[l].density_normal = outs[l].density_normal ? outs[l].density_normal + off * n : nullptr;
       dump.act[l] = s.act[l], dump.v[l] = s.v[l], dump.raw_rgb[l] = s.raw_rgb[l], dump.raw_density[l] = s.raw_density[l];
     }
+    dump.rng_state = rng_state;
     CUDA_TRY(mipnerf::tc_forward(cfg, &wl, &rc_, randomized, t_rand ? t_rand + off * (n + 1) : nullptr,
                                  u_jitter ? u_jitter + off * (n + 1) : nullptr, rng, white_bkgd, precision, lo, s.tcws,
                                  s.tcws_bytes, st, &dump, off));
@@ -643,7 +644,8 @@ static int forward_backward_impl(const mipnerf_b200_config* cfg, const mipnerf_b
                                  const float* u_jitter, const mipnerf_b200_rng* rng, int white_bkgd, int precision,
                                  const mipnerf_b200_loss* loss, mipnerf_b200_level_out* outs,
                                  const mipnerf_b200_linear_grad* grads, int num_grads, int accumulate,
-                                 void* workspace, size_t workspace_bytes, void* stream) {
+                                 void* workspace, size_t workspace_bytes, void* stream,
+                                 const uint64_t* rng_state = nullptr) {
   Dims d;
   int rc;
   if ((rc = check_config(cfg, &d))) return rc;
@@ -694,9 +696,14 @@ static int forward_backward_impl(const mipnerf_b200_config* cfg, const mipnerf_b
 
   {
     const char* fused_env = getenv("MIPNERF_B200_TRAIN_FUSED");
-    if (tc && B > 0 && train_fused_supported(cfg, precision) && !(fused_env && fused_env[0] == '0'))
+    const bool fused = tc && train_fused_supported(cfg, precision) && !(fused_env && fused_env[0] == '0');
+    if (rng_state && !fused)
+      return fail(MIPNERF_B200_EUNSUPPORTED,
+                  "rng_state: the fused BF16 / FP16 training step only (default architecture, "
+                  "MIPNERF_B200_TRAIN_FUSED unset)");
+    if (fused && B > 0)
       return forward_backward_fused(cfg, d, w, rays, randomized, t_rand, u_jitter, rng, white_bkgd, precision, loss, outs,
-                                    grads, touched, workspace, st);
+                                    grads, touched, workspace, st, rng_state);
   }
   // ---- tensor-core mode: B operands of every forward / dgrad GEMM, packed once per call (the weights change every
   //      optimiser step).  fwd[i] = W_i[:, :k_main], fwd_skip[i] = W_i[:, 256:352], bwd[i] = W_i[:, :256]^T;
@@ -885,6 +892,17 @@ int mipnerf_b200_forward_backward_rng(const mipnerf_b200_config* cfg, const mipn
                                accumulate, workspace, workspace_bytes, stream);
 }
 
+int mipnerf_b200_forward_backward_rng_state(const mipnerf_b200_config* cfg, const mipnerf_b200_weights* w,
+                                            const mipnerf_b200_rays* rays, const uint64_t* rng_state, int white_bkgd,
+                                            int precision, const mipnerf_b200_loss* loss, mipnerf_b200_level_out* outs,
+                                            const mipnerf_b200_linear_grad* grads, int num_grads, int accumulate,
+                                            void* workspace, size_t workspace_bytes, void* stream) {
+  if (!rng_state) return fail(MIPNERF_B200_EINVAL, "rng_state is NULL");
+  const mipnerf_b200_rng placeholder = {0, 0};  // selects the in-kernel draws; the kernel reads rng_state instead
+  return forward_backward_impl(cfg, w, rays, 1, nullptr, nullptr, &placeholder, white_bkgd, precision, loss, outs, grads,
+                               num_grads, accumulate, workspace, workspace_bytes, stream, rng_state);
+}
+
 int mipnerf_b200_linear_tc(const float* x, const float* weight, const float* bias, float* y, int64_t m, int n,
                            int k, int relu, int precision, void* scratch, size_t scratch_bytes, void* stream) {
   if (m < 0 || !mipnerf::linear_tc_shape_ok(n, k))
@@ -955,6 +973,54 @@ int mipnerf_b200_adam_step_multi(int count, float* const* params, const float* c
     CUDA_TRY(mipnerf::launch_adam_multi(t, (float)beta1, (float)beta2, (float)eps, (float)(lr / bc1), (float)sqrt(bc2),
                                         (float)grad_scale, (cudaStream_t)stream));
   }
+  return MIPNERF_B200_OK;
+}
+
+int mipnerf_b200_adam_step_multi_table(int count, float* const* params, const float* const* grads,
+                                       float* const* exp_avg, float* const* exp_avg_sq, const int64_t* sizes,
+                                       const float* step_size, const float* bc2_sqrt, int64_t table_len,
+                                       const int64_t* step, double beta1, double beta2, double eps, double grad_scale,
+                                       void* stream) {
+  if (count < 0 || table_len < 2) return fail(MIPNERF_B200_EINVAL, "bad count / table_len");
+  if (count > 0 && (!params || !grads || !exp_avg || !exp_avg_sq || !sizes || !step_size || !bc2_sqrt || !step))
+    return fail(MIPNERF_B200_EINVAL, "NULL array");
+  for (int base = 0; base < count; base += mipnerf::kAdamMaxTensors) {
+    mipnerf::AdamMulti t{};
+    t.count = (count - base) < mipnerf::kAdamMaxTensors ? (count - base) : mipnerf::kAdamMaxTensors;
+    for (int k = 0; k < t.count; ++k) {
+      const int i = base + k;
+      if (sizes[i] < 0 || (sizes[i] > 0 && (!params[i] || !grads[i] || !exp_avg[i] || !exp_avg_sq[i])))
+        return fail(MIPNERF_B200_EINVAL, "tensor %d: NULL pointer or negative size", i);
+      t.p[k] = params[i], t.g[k] = grads[i], t.m[k] = exp_avg[i], t.v[k] = exp_avg_sq[i], t.n[k] = sizes[i];
+      t.blocks[k] = (int)((sizes[i] + 255) / 256);
+    }
+    CUDA_TRY(mipnerf::launch_adam_multi_table(t, (float)beta1, (float)beta2, (float)eps, step_size, bc2_sqrt, table_len,
+                                              step, (float)grad_scale, (cudaStream_t)stream));
+  }
+  return MIPNERF_B200_OK;
+}
+
+int mipnerf_b200_train_step_advance(int64_t* step, uint64_t* rng_state, const float* loss, const float* psnr,
+                                    float* ring, int ring_len, void* stream) {
+  if (!step || !rng_state) return fail(MIPNERF_B200_EINVAL, "step / rng_state is NULL");
+  if (ring_len < 0 || (ring_len > 0 && (!ring || !loss || !psnr))) return fail(MIPNERF_B200_EINVAL, "bad ring");
+  CUDA_TRY(mipnerf::launch_train_step_advance(step, rng_state, loss, psnr, ring, ring_len, (cudaStream_t)stream));
+  return MIPNERF_B200_OK;
+}
+
+int mipnerf_b200_sample_pixels(const float* cam_table, const int64_t* offsets, const int32_t* widths, int num_images,
+                               int64_t num_pixels, const uint64_t* rng_state, int64_t ray_base, int64_t count,
+                               const float* atlas, int64_t* pixel_ids, float* origins, float* directions,
+                               float* viewdirs, float* radii, float* lossmult, float* near_out, float* far_out,
+                               float* rgb, void* stream) {
+  if (num_images < 1 || num_pixels < 1 || num_pixels > ((int64_t)1 << 32) || count < 0 || ray_base < 0)
+    return fail(MIPNERF_B200_EINVAL, "bad num_images / num_pixels (1 .. 2^32) / count / ray_base");
+  if (count > 0 && (!cam_table || !offsets || !widths || !atlas || !rng_state || !origins || !directions || !viewdirs ||
+                    !radii || !lossmult || !near_out || !far_out))
+    return fail(MIPNERF_B200_EINVAL, "NULL tensor");
+  CUDA_TRY(mipnerf::launch_sample_pixels(cam_table, offsets, widths, num_images, num_pixels, rng_state, ray_base, count,
+                                         atlas, pixel_ids, origins, directions, viewdirs, radii, lossmult, near_out,
+                                         far_out, rgb, (cudaStream_t)stream));
   return MIPNERF_B200_OK;
 }
 

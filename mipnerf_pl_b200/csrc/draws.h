@@ -14,6 +14,7 @@ struct Draws {
   float scale;         // u_jitter: 1/num_samples - eps (uniform_(to=...)); t_rand: 1; density normals: density_noise
 };
 constexpr int kDensityNoiseStream = 32;  // + level (models/mip_nerf.py:232-233)
+constexpr int kPixelStream = 64;         // training batch: the pixel ids of mipnerf_b200_sample_pixels
 __host__ __device__ __forceinline__ Draws draws_from_array(const float* ptr) {
   Draws d{};
   d.ptr = ptr;
@@ -27,6 +28,22 @@ __host__ __device__ __forceinline__ Draws draws_philox(uint64_t seed, uint64_t o
                                                        float scale) {
   Draws d{};
   d.seed = seed, d.offset = offset, d.ray_base = ray_base, d.stream = stream, d.philox = 1, d.scale = scale;
+  return d;
+}
+
+// `d` with (seed, offset) read from the device array `state` when the kernel runs (a captured training step replays
+// the same kernel parameters and still draws fresh numbers), if d draws in-kernel and state is set; kDevice = false
+// compiles to `d` itself.  The pointer travels next to the Draws (LevelParams::rng_state), not inside them: a larger
+// Draws would move the parameter offsets of every inference kernel and with them their code.
+template <bool kDevice>
+__device__ __forceinline__ Draws draws_at_state(const Draws& d, const uint64_t* state) {
+  if constexpr (kDevice) {
+    if (state && d.philox && !d.ptr) {
+      Draws r = d;
+      r.seed = state[0], r.offset = state[1];
+      return r;
+    }
+  }
   return d;
 }
 

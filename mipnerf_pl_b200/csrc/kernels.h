@@ -19,6 +19,11 @@ cudaError_t launch_rays_from_pixels(const float* cam_table, const int64_t* offse
                                     int num_images, const int64_t* pixel_ids, int64_t count, const float* atlas,
                                     float* origins, float* directions, float* viewdirs, float* radii,
                                     float* lossmult, float* near_o, float* far_o, float* rgb, cudaStream_t st);
+cudaError_t launch_sample_pixels(const float* cam_table, const int64_t* offsets, const int32_t* widths, int num_images,
+                                 int64_t num_pixels, const uint64_t* rng_state, int64_t ray_base, int64_t count,
+                                 const float* atlas, int64_t* pixel_ids, float* origins, float* directions,
+                                 float* viewdirs, float* radii, float* lossmult, float* near_o, float* far_o, float* rgb,
+                                 cudaStream_t st);
 cudaError_t launch_coarse_t(const float* near, const float* far, const Draws& t_rand, float* t_out,
                             int64_t num_rays, int n, int randomized, int disparity, cudaStream_t st);
 cudaError_t launch_philox_uniform(const Draws& d, float* out, int64_t num_rays, int ncols, cudaStream_t st);
@@ -87,6 +92,12 @@ struct AdamMulti {  // passed by value in the kernel parameters
 };
 cudaError_t launch_adam_multi(const AdamMulti& t, float beta1, float beta2, float eps, float step_size, float bc2_sqrt,
                               float grad_scale, cudaStream_t st);
+// the same update with lr / bc1 and sqrt(bc2) read from per-step tables at the device step count *step + 1
+cudaError_t launch_adam_multi_table(const AdamMulti& t, float beta1, float beta2, float eps, const float* step_size,
+                                    const float* bc2_sqrt, int64_t table_len, const int64_t* step, float grad_scale,
+                                    cudaStream_t st);
+cudaError_t launch_train_step_advance(int64_t* step, uint64_t* rng_state, const float* loss, const float* psnr,
+                                      float* ring, int ring_len, cudaStream_t st);
 
 // ---- linear_tc.cu (tcgen05 linear layer for the training step's forward / dgrad GEMMs) ----
 size_t linear_tc_image_bytes(int n, int k);

@@ -202,6 +202,8 @@ struct LevelParams {
   int disable_integration;
   float density_bias, rgb_scale, rgb_padding;
   Draws dnoise;  // density noise of randomized mode (models/mip_nerf.py:232-233): normals [B,128] or in-kernel; scale = std
+  const uint64_t* rng_state;  // training forward, nullable: device (seed, offset) of the in-kernel draws (last member:
+                              // the inference kernels' parameter offsets stay where they were)
 };
 
 // raw density of (ray, row) with the density noise added; kept out of line so that the (default) noise-free
@@ -920,11 +922,13 @@ __global__ void __launch_bounds__(kThreads, 1) mlp_level_kernel(const LevelParam
         // coarse fenceposts (bit-identical to coarse_t_kernel)
         const float nr = __ldg(p.near + ray), fr = __ldg(p.far + ray);
         const bool jit = draws_active(p.t_rand);
+        const Draws t_rand = draws_at_state<kTrain>(p.t_rand, p.rng_state);
         for (int j = lane; j <= kN; j += 32)
           __stcg(t_ray + j, coarse_fencepost(nr, fr, j, kN, p.disparity, jit,
-                                             jit ? draw_uniform(p.t_rand, ray, j, kN + 1) : 0.f));
+                                             jit ? draw_uniform(t_rand, ray, j, kN + 1) : 0.f));
       } else if (p.t_mode == 2 && early_scratch) {
-        resample_warp_lean<true>(p.t_prev + ray * (kN + 1), p.w_prev + ray * kN, kN, kN + 1, p.randomized, p.u_jitter,
+        resample_warp_lean<true>(p.t_prev + ray * (kN + 1), p.w_prev + ray * kN, kN, kN + 1, p.randomized,
+                                 draws_at_state<kTrain>(p.u_jitter, p.rng_state),
                                  ray, p.resample_padding, early_scratch, t_ray,
                                  p.inds ? p.inds + ray * (kN + 1) : nullptr, lane);
       }
@@ -971,8 +975,9 @@ __global__ void __launch_bounds__(kThreads, 1) mlp_level_kernel(const LevelParam
       TRACE(EV(3, 0, 0, slot));
       if (p.t_mode == 2 && !early_scratch) {
         // no spare shared memory: the feature tile this warp is about to fill doubles as the scratch
-        resample_warp_lean<true>(p.t_prev + ray * (kN + 1), p.w_prev + ray * kN, kN, kN + 1, p.randomized, p.u_jitter,
-                                 ray, p.resample_padding, reinterpret_cast<float*>(myF), t_ray,
+        resample_warp_lean<true>(p.t_prev + ray * (kN + 1), p.w_prev + ray * kN, kN, kN + 1, p.randomized,
+                                 draws_at_state<kTrain>(p.u_jitter, p.rng_state), ray, p.resample_padding,
+                                 reinterpret_cast<float*>(myF), t_ray,
                                  p.inds ? p.inds + ray * (kN + 1) : nullptr, lane);
         __threadfence_block();
         __syncwarp();
@@ -1178,7 +1183,8 @@ __global__ void __launch_bounds__(kThreads, 1) mlp_level_kernel(const LevelParam
       }
       float raw_dens = dens + c_small.b_density;
       if (kNoise || kTrain) {  // models/mip_nerf.py:232-233 (randomized and density_noise > 0)
-        if (draws_active(p.dnoise) && valid) raw_dens = noisy_raw_density(raw_dens, p.dnoise, ray, row);
+        if (draws_active(p.dnoise) && valid)
+          raw_dens = noisy_raw_density(raw_dens, draws_at_state<kTrain>(p.dnoise, p.rng_state), ray, row);
       }
       if (kTrain && valid) {  // training: the raw heads as well (render_backward recomputes the rest; the density
         const int64_t sidx = ray * kN + row;  // head WITH its noise, so that softplus' is taken at the same point)
@@ -2268,6 +2274,7 @@ cudaError_t tc_forward(const mipnerf_b200_config* c, const mipnerf_b200_weights*
       p.density_bias = c->density_bias, p.rgb_scale = rgb_scale, p.rgb_padding = c->rgb_padding;
       p.dnoise = density_noise_draws(c, randomized, outs[l].density_normal, rng, off, l, kN);
       if (!outs[l].density_normal) p.dnoise.ray_base += ray_base;
+      p.rng_state = dump ? dump->rng_state : nullptr;
       e = launch_level(p, precision, st);
       if (e != cudaSuccess) return e;
       t_prev = t_cur;

@@ -25,6 +25,7 @@ struct TcTrainDump {
   uint8_t* v[2];          // [rays][32 KB]: view-layer output (post-ReLU)
   float* raw_rgb[2];      // [rays,128,3]
   float* raw_density[2];  // [rays,128]
+  const uint64_t* rng_state;  // nullable: device (seed, offset) of the in-kernel draws, read when the kernel runs
 };
 cudaError_t tc_forward(const mipnerf_b200_config* cfg, const mipnerf_b200_weights* w,
                        const mipnerf_b200_rays* rays, int randomized, const float* t_rand,

@@ -329,20 +329,13 @@ __global__ void generate_rays_kernel(const Pose c, int height, int width, float 
 //   radius = |R . pix2cam[:,1]| * 2/sqrt(12)   (the y-neighbour distance of the reference, which is the same
 //   vector for every pixel of an image; see generate_rays_kernel for why it is evaluated analytically).
 // ---------------------------------------------------------------------------------------------
-__global__ void rays_from_pixels_kernel(const float* __restrict__ cam_table, const int64_t* __restrict__ offsets,
-                                        const int32_t* __restrict__ widths, int num_images,
-                                        const int64_t* __restrict__ pixel_ids, int64_t count,
-                                        const float* __restrict__ atlas, float* __restrict__ origins,
-                                        float* __restrict__ directions, float* __restrict__ viewdirs,
-                                        float* __restrict__ radii, float* __restrict__ lossmult,
-                                        float* __restrict__ near_o, float* __restrict__ far_o,
-                                        float* __restrict__ rgb) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= count) return;
-  // ids outside the atlas are clamped to its first / last row (never read out of bounds); offsets[num_images] = P
-  const int64_t total = __ldg(offsets + num_images);
-  int64_t id = __ldg(pixel_ids + i);
-  id = id < 0 ? 0 : (id >= total ? total - 1 : id);
+__device__ __forceinline__ void ray_from_pixel(const float* __restrict__ cam_table, const int64_t* __restrict__ offsets,
+                                               const int32_t* __restrict__ widths, int num_images, int64_t i,
+                                               int64_t id, const float* __restrict__ atlas,
+                                               float* __restrict__ origins, float* __restrict__ directions,
+                                               float* __restrict__ viewdirs, float* __restrict__ radii,
+                                               float* __restrict__ lossmult, float* __restrict__ near_o,
+                                               float* __restrict__ far_o, float* __restrict__ rgb) {
   int lo = 0, hi = num_images;  // offsets[lo] <= id < offsets[hi]
   while (hi - lo > 1) {
     const int mid = (lo + hi) >> 1;
@@ -382,6 +375,51 @@ __global__ void rays_from_pixels_kernel(const float* __restrict__ cam_table, con
   }
 }
 
+__global__ void rays_from_pixels_kernel(const float* __restrict__ cam_table, const int64_t* __restrict__ offsets,
+                                        const int32_t* __restrict__ widths, int num_images,
+                                        const int64_t* __restrict__ pixel_ids, int64_t count,
+                                        const float* __restrict__ atlas, float* __restrict__ origins,
+                                        float* __restrict__ directions, float* __restrict__ viewdirs,
+                                        float* __restrict__ radii, float* __restrict__ lossmult,
+                                        float* __restrict__ near_o, float* __restrict__ far_o,
+                                        float* __restrict__ rgb) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= count) return;
+  // ids outside the atlas are clamped to its first / last row (never read out of bounds); offsets[num_images] = P
+  const int64_t total = __ldg(offsets + num_images);
+  int64_t id = __ldg(pixel_ids + i);
+  id = id < 0 ? 0 : (id >= total ? total - 1 : id);
+  ray_from_pixel(cam_table, offsets, widths, num_images, i, id, atlas, origins, directions, viewdirs, radii, lossmult,
+                 near_o, far_o, rgb);
+}
+
+// A uniformly random training batch drawn on the device: pixel id of ray i = floor(x * P / 2^32), x the first 32-bit
+// Philox4x32-10 output of counter (ray_base + i, stream kPixelStream << 24, offset) under key (seed, offset) read
+// from `rng_state` when the kernel runs -- the counter layout of draw_uniform, so mipnerf_b200_philox_uniform's
+// generator (and its host mirror) reproduces the ids.  Each id is hit by floor or ceil of 2^32 / P of the 2^32
+// draws: its probability differs from 1/P by less than 2^-32.
+__global__ void sample_pixels_kernel(const float* __restrict__ cam_table, const int64_t* __restrict__ offsets,
+                                     const int32_t* __restrict__ widths, int num_images, uint64_t num_pixels,
+                                     const uint64_t* __restrict__ rng_state, int64_t ray_base, int64_t count,
+                                     const float* __restrict__ atlas, int64_t* __restrict__ pixel_ids,
+                                     float* __restrict__ origins, float* __restrict__ directions,
+                                     float* __restrict__ viewdirs, float* __restrict__ radii,
+                                     float* __restrict__ lossmult, float* __restrict__ near_o,
+                                     float* __restrict__ far_o, float* __restrict__ rgb) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= count) return;
+  const uint64_t seed = rng_state[0], offset = rng_state[1];
+  const uint64_t g = (uint64_t)(ray_base + i);
+  const uint32_t x = philox4x32_10_first((uint32_t)g, (uint32_t)(g >> 32), (uint32_t)kPixelStream << 24,
+                                         (uint32_t)offset, (uint32_t)seed, (uint32_t)(seed >> 32) ^ (uint32_t)(offset >> 32));
+  int64_t id = (int64_t)(((uint64_t)x * num_pixels) >> 32);  // num_pixels <= 2^32: id < num_pixels
+  const int64_t total = __ldg(offsets + num_images);          // never past the atlas, whatever num_pixels says
+  id = id < total ? id : total - 1;
+  if (pixel_ids) pixel_ids[i] = id;
+  ray_from_pixel(cam_table, offsets, widths, num_images, i, id, atlas, origins, directions, viewdirs, radii, lossmult,
+                 near_o, far_o, rgb);
+}
+
 // ---------------------------------------------------------------------------------------------
 // launchers
 // ---------------------------------------------------------------------------------------------
@@ -394,6 +432,20 @@ cudaError_t launch_rays_from_pixels(const float* cam_table, const int64_t* offse
   rays_from_pixels_kernel<<<blocks_for(count, 256), 256, 0, st>>>(cam_table, offsets, widths, num_images, pixel_ids,
                                                                  count, atlas, origins, directions, viewdirs, radii,
                                                                  lossmult, near_o, far_o, rgb);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_sample_pixels(const float* cam_table, const int64_t* offsets, const int32_t* widths, int num_images,
+                                 int64_t num_pixels, const uint64_t* rng_state, int64_t ray_base, int64_t count,
+                                 const float* atlas, int64_t* pixel_ids, float* origins, float* directions,
+                                 float* viewdirs, float* radii, float* lossmult, float* near_o, float* far_o, float* rgb,
+                                 cudaStream_t st) {
+  if (count == 0) return cudaSuccess;
+  LaunchScope scope(kKernRayGen, st);
+  sample_pixels_kernel<<<blocks_for(count, 256), 256, 0, st>>>(cam_table, offsets, widths, num_images,
+                                                              (uint64_t)num_pixels, rng_state, ray_base, count, atlas,
+                                                              pixel_ids, origins, directions, viewdirs, radii, lossmult,
+                                                              near_o, far_o, rgb);
   return cudaGetLastError();
 }
 

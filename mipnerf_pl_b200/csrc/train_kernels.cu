@@ -567,6 +567,60 @@ cudaError_t launch_adam_multi(const AdamMulti& t, float beta1, float beta2, floa
   return cudaGetLastError();
 }
 
+// adam_multi_kernel for a captured training step: the step count lives on the device, and lr / bc1, sqrt(bc2) come
+// from tables the host filled with the double-precision math of mipnerf_b200_adam_step_multi (entry t = step t).
+__global__ void adam_multi_table_kernel(const AdamMulti t, float beta1, float beta2, float eps,
+                                        const float* __restrict__ step_size_tab, const float* __restrict__ bc2_sqrt_tab,
+                                        int64_t table_len, const int64_t* __restrict__ step, float grad_scale) {
+  int b = blockIdx.x, k = 0;
+  while (k + 1 < t.count && b >= t.blocks[k]) b -= t.blocks[k++];
+  const int64_t i = (int64_t)b * blockDim.x + threadIdx.x;
+  if (i >= t.n[k]) return;
+  int64_t s = *step + 1;
+  s = s < 1 ? 1 : (s >= table_len ? table_len - 1 : s);  // never read outside the tables (the host sizes them)
+  const float step_size = step_size_tab[s], bc2_sqrt = bc2_sqrt_tab[s];
+  float* __restrict__ p = t.p[k];
+  float* __restrict__ m = t.m[k];
+  float* __restrict__ v = t.v[k];
+  const float gi = __fmul_rn(t.g[k][i], grad_scale);
+  const float mi = __fadd_rn(m[i], __fmul_rn(__fsub_rn(gi, m[i]), 1.0f - beta1));
+  const float vi = __fadd_rn(__fmul_rn(v[i], beta2), __fmul_rn(__fmul_rn(gi, gi), 1.0f - beta2));
+  m[i] = mi;
+  v[i] = vi;
+  const float denom = __fadd_rn(__fdiv_rn(sqrtf(vi), bc2_sqrt), eps);
+  p[i] = __fadd_rn(p[i], __fmul_rn(-step_size, __fdiv_rn(mi, denom)));
+}
+
+// End of a captured training step: log (loss, psnr) into ring row step % ring_len, then step += 1 and the Philox
+// offset += 1 (one fresh set of draws per step, like MipNerf.next_rng).  One thread; runs after every reader.
+__global__ void train_step_advance_kernel(int64_t* step, uint64_t* rng_state, const float* loss, const float* psnr,
+                                          float* ring, int ring_len) {
+  const int64_t s = *step;
+  if (ring_len > 0) {
+    ring[(s % ring_len) * 2 + 0] = *loss;
+    ring[(s % ring_len) * 2 + 1] = *psnr;
+  }
+  *step = s + 1;
+  rng_state[1] += 1;
+}
+
+cudaError_t launch_adam_multi_table(const AdamMulti& t, float beta1, float beta2, float eps, const float* step_size,
+                                    const float* bc2_sqrt, int64_t table_len, const int64_t* step, float grad_scale,
+                                    cudaStream_t st) {
+  int total = 0;
+  for (int k = 0; k < t.count; ++k) total += t.blocks[k];
+  if (total == 0) return cudaSuccess;
+  LaunchScope scope(kKernAdam, st);
+  adam_multi_table_kernel<<<total, 256, 0, st>>>(t, beta1, beta2, eps, step_size, bc2_sqrt, table_len, step, grad_scale);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_train_step_advance(int64_t* step, uint64_t* rng_state, const float* loss, const float* psnr,
+                                      float* ring, int ring_len, cudaStream_t st) {
+  train_step_advance_kernel<<<1, 1, 0, st>>>(step, rng_state, loss, psnr, ring, ring_len);
+  return cudaGetLastError();
+}
+
 cudaError_t launch_adam(float* p, const float* g, float* m, float* v, int64_t n, float beta1, float beta2,
                         float eps, float step_size, float bc2_sqrt, float grad_scale, cudaStream_t st) {
   if (n == 0) return cudaSuccess;

@@ -269,6 +269,50 @@ class DeviceRayBank:
         ids = torch.randint(0, self.num_pixels, (batch_size,), device=self.device, generator=generator)
         return self.rays(ids)
 
+    def sample_philox(self, rng_state: torch.Tensor, batch_size: int, ray_base: int = 0, out=None):
+        """A uniformly random batch drawn by ONE kernel from the Philox state `rng_state` (int64 [2] on this device: seed,
+        offset, read when the kernel runs -- so a CUDA graph replays it with fresh ids once the offset moves).
+        Returns (Rays, rgb, pixel_ids); `out` = such a triple to write into.  `philox_pixel_ids` recomputes the ids."""
+        from . import _cabi
+        from .ops import _stream
+        if out is None:
+            mk = lambda c: torch.empty(batch_size, c, device=self.device)  # noqa: E731
+            out = (Rays(mk(3), mk(3), mk(3), mk(1), mk(1), mk(1), mk(1)), mk(3),
+                   torch.empty(batch_size, dtype=torch.int64, device=self.device))
+        r, rgb, ids = out
+        with torch.cuda.device(self.device):
+            _cabi.check(_cabi.lib().mipnerf_b200_sample_pixels(
+                self.cam_table.data_ptr(), self.offsets.data_ptr(), self.widths.data_ptr(), self.num_images,
+                self.num_pixels, rng_state.data_ptr(), int(ray_base), batch_size, self.atlas.data_ptr(), ids.data_ptr(),
+                *[f.data_ptr() for f in r], rgb.data_ptr(), _stream(self.device)), "sample_pixels")
+        return out
+
+
+def philox_pixel_ids(seed: int, offset: int, count: int, num_pixels: int, ray_base: int = 0) -> np.ndarray:
+    """Host mirror of mipnerf_b200_sample_pixels' ids: Philox4x32-10 (the generator of the in-kernel draws,
+    mipnerf_b200_philox_uniform) on counter (ray_base + i, 64 << 24, offset), key (seed, offset), first output word x;
+    id = (x * num_pixels) >> 32."""
+    seed &= (1 << 64) - 1
+    offset &= (1 << 64) - 1
+    g = np.arange(ray_base, ray_base + count, dtype=np.uint64)
+    x = philox4x32_10_first(g & 0xFFFFFFFF, g >> np.uint64(32), 64 << 24, offset & 0xFFFFFFFF,
+                            seed & 0xFFFFFFFF, (seed >> 32) ^ (offset >> 32))
+    return ((x.astype(np.uint64) * np.uint64(num_pixels)) >> np.uint64(32)).astype(np.int64)
+
+
+def philox4x32_10_first(c0, c1, c2, c3, k0, k1) -> np.ndarray:
+    """First output word of Philox4x32-10 (ray_math.cuh), vectorised over the counter words."""
+    m = np.uint64(0xFFFFFFFF)
+    n = np.broadcast(c0, c1, c2, c3).shape
+    c = [np.broadcast_to(np.asarray(v, dtype=np.uint64), n).copy() for v in (c0, c1, c2, c3)]
+    k0, k1 = np.uint64(k0), np.uint64(k1)
+    for _ in range(10):
+        p0, p1 = np.uint64(0xD2511F53) * c[0], np.uint64(0xCD9E8D57) * c[2]
+        hi0, lo0, hi1, lo1 = p0 >> np.uint64(32), p0 & m, p1 >> np.uint64(32), p1 & m
+        c = [hi1 ^ c[1] ^ k0, lo1, hi0 ^ c[3] ^ k1, lo0]
+        k0, k1 = (k0 + np.uint64(0x9E3779B9)) & m, (k1 + np.uint64(0xBB67AE85)) & m
+    return c[0].astype(np.uint32)
+
 
 def write_synthetic_blender_scene(root: str, n_images: int = 3, height: int = 16, width: int = 12, seed: int = 0,
                                   splits: Sequence[str] = ("train", "val", "test")) -> None:

@@ -10,6 +10,8 @@ tcgen05 with 16-bit operands and fp32 accumulation, wgrad / heads / rendering in
 * `FusedAdam`             torch.optim.Adam semantics, update done by `mipnerf_b200_adam_step`.
 * `MipLRDecay`, `mip_lr`  utils/lr_schedule.py:51-60 (log-linear decay with the delayed warm-up).
 * `allreduce_grads`       DDP's gradient all-reduce over the ray shards: ONE collective on a flat buffer.
+* `adam_tables`           the per-step (lr/bc1, sqrt(bc2)) of FusedAdam + MipLRDecay for the captured training step
+                          (graph.GraphedTrainStep), computed with the host math FusedAdam hands the library.
 
 Gradients do not flow into the fenceposts (stop_resample_grad=True, the reference default); a model built
 with stop_resample_grad=False is refused rather than silently trained with different gradients.
@@ -175,6 +177,23 @@ def allreduce_grads(params: Iterable[torch.Tensor], group=None, average: bool = 
         off += g.numel()
 
 
+def adam_tables(num_steps: int, betas, lr_init: float, lr_final: float, max_steps: int, lr_delay_steps: int = 0,
+                lr_delay_mult: float = 1.0):
+    """float32 tables (step_size, bc2_sqrt) of length num_steps + 1: entry t (t >= 1) is what update t of FusedAdam
+    stepped with MipLRDecay uses -- lr = mip_lr(t - 1) (the scheduler has stepped t - 1 times), bc1 = 1 - b1^t,
+    bc2 = 1 - b2^t in double, then (float)(lr / bc1) and (float)sqrt(bc2) as mipnerf_b200_adam_step_multi rounds
+    them.  Entry 0 is unused."""
+    import numpy as np
+    b1, b2 = float(betas[0]), float(betas[1])
+    step_size = np.zeros(num_steps + 1, dtype=np.float32)
+    bc2_sqrt = np.ones(num_steps + 1, dtype=np.float32)
+    for t in range(1, num_steps + 1):
+        lr = mip_lr(t - 1, lr_init, lr_final, max_steps, lr_delay_steps, lr_delay_mult)
+        step_size[t] = np.float32(lr / (1.0 - math.pow(b1, float(t))))
+        bc2_sqrt[t] = np.float32(math.sqrt(1.0 - math.pow(b2, float(t))))
+    return step_size, bc2_sqrt
+
+
 def _level_multipliers(num_levels: int, coarse_loss_mult: float, dist_mult: float):
     """loss = coarse_loss_mult * (mse_coarse + 0.01 dist_coarse) + mse_fine + 0.01 dist_fine
     (models/nerf_system.py:110-111; every level before the last counts as coarse)."""
@@ -185,7 +204,11 @@ def _level_multipliers(num_levels: int, coarse_loss_mult: float, dist_mult: floa
 
 def _run(model: MipNerf, rays: Rays, rgbs: torch.Tensor, randomized: bool, white_bkgd: bool,
          coarse_loss_mult: float, dist_mult: float, disable_multiscale_loss: bool, t_rand, u_jitter,
-         grad_tensors: Sequence[torch.Tensor], accumulate: bool, mask_sum, global_rays, density_normal=None):
+         grad_tensors: Sequence[torch.Tensor], accumulate: bool, mask_sum, global_rays, density_normal=None,
+         rng_state: Optional[torch.Tensor] = None, level_mults=None):
+    """`rng_state` (int64 [2] on the device, read as uint64 seed / offset by the kernels) replaces `model.next_rng()`
+    for randomized=True; `level_mults` = (mse, dist) multipliers [levels] already on the device.  Both exist so that
+    the call can be captured into a CUDA graph (no host-to-device copy, no host-side state)."""
     if not model.stop_resample_grad:
         raise NotImplementedError("training kernels implement stop_resample_grad=True (the reference default)")
     prec = _cabi.PRECISIONS[model.precision]   # fp32: the parity mode; bf16 / fp16: forward + dgrad GEMMs on tcgen05
@@ -200,7 +223,9 @@ def _run(model: MipNerf, rays: Rays, rgbs: torch.Tensor, randomized: bool, white
     rng = None
     noisy = bool(randomized) and model.density_noise > 0    # models/mip_nerf.py:232-233
     normals = [None] * levels
-    if randomized and t_rand is None and u_jitter is None and density_normal is None:
+    if randomized and rng_state is not None:
+        pass                            # (seed, offset) read from the device when the kernels run
+    elif randomized and t_rand is None and u_jitter is None and density_normal is None:
         rng = model.next_rng()          # uniforms / normals drawn inside the kernels (Philox), as every training step does
     elif randomized:
         t_rand = _f32(t_rand) if t_rand is not None else draw_t_rand(b, n, dev)
@@ -244,16 +269,27 @@ def _run(model: MipNerf, rays: Rays, rgbs: torch.Tensor, randomized: bool, white
     tail = (int(bool(white_bkgd)), prec, C.byref(loss), outs, garr, len(lins), int(bool(accumulate)),
             scratch.data_ptr() if nbytes else None, scratch.numel() if nbytes else 0, _stream(dev))
     with torch.cuda.device(dev):
-        if rng is not None:
+        if randomized and rng_state is not None:
+            rc = lib.mipnerf_b200_forward_backward_rng_state(C.byref(cfg), C.byref(ws), C.byref(rs), rng_state.data_ptr(),
+                                                             *tail)
+        elif rng is not None:
             rc = lib.mipnerf_b200_forward_backward_rng(C.byref(cfg), C.byref(ws), C.byref(rs), C.byref(rng), *tail)
         else:
             rc = lib.mipnerf_b200_forward_backward(C.byref(cfg), C.byref(ws), C.byref(rs), int(bool(randomized)),
                                                    _ptr(t_rand), _ptr(u_jitter), *tail)
         _cabi.check(rc, "forward_backward")
+    if level_mults is None:
+        level_mults = (torch.tensor(mse_m, device=dev), torch.tensor(dist_m, device=dev))
+    mse, distl, total = _assemble_loss(sqerr, dl, mask_sum, global_rays, *level_mults)
+    return {"loss": total, "mse": mse, "distloss": distl, "ret": ret}
+
+
+def _assemble_loss(sqerr, dl, mask_sum, global_rays: int, mse_mult: torch.Tensor, dist_mult: torch.Tensor):
+    """(mse [levels], distloss [levels], loss) from the per-ray terms the step leaves behind; device ops only."""
     mse = sqerr.sum(dim=1) / mask_sum                      # [levels]   (models/nerf_system.py:104-105)
     distl = dl.sum(dim=1) / max(global_rays, 1)            # [levels]   (:106)
-    total = (mse * torch.tensor(mse_m, device=dev) + distl * torch.tensor(dist_m, device=dev)).sum()
-    return {"loss": total, "mse": mse, "distloss": distl, "ret": ret}
+    total = (mse * mse_mult + distl * dist_mult).sum()
+    return mse, distl, total
 
 
 def _param_list(model: MipNerf) -> List[torch.nn.Parameter]:
@@ -267,6 +303,13 @@ def forward_backward(model: MipNerf, rays: Rays, rgbs: torch.Tensor, randomized:
     """Forward + backward of the training loss; gradients are written (or added, with `accumulate`)
     into `param.grad`.  For a ray shard of a larger batch pass the GLOBAL `mask_sum` / `global_rays`;
     shard gradients then sum to the full-batch gradient."""
+    params = _grads_ready(model)
+    return _run(model, rays, rgbs, randomized, white_bkgd, coarse_loss_mult, dist_mult, disable_multiscale_loss,
+                t_rand, u_jitter, [p.grad for p in params], accumulate, mask_sum, global_rays, density_normal)
+
+
+def _grads_ready(model: MipNerf) -> List[torch.nn.Parameter]:
+    """The MLP's parameters, each with a contiguous `.grad` (carved from one flat buffer on first use)."""
     params = _param_list(model)
     if all(p.grad is None for p in params) and len({(p.device, p.dtype) for p in params}) == 1:
         # first step: carve every .grad out of ONE flat buffer, so that the data-parallel all-reduce
@@ -281,8 +324,7 @@ def forward_backward(model: MipNerf, rays: Rays, rgbs: torch.Tensor, randomized:
             p.grad = torch.zeros_like(p)
         elif not p.grad.is_contiguous():
             p.grad = p.grad.contiguous()
-    return _run(model, rays, rgbs, randomized, white_bkgd, coarse_loss_mult, dist_mult, disable_multiscale_loss,
-                t_rand, u_jitter, [p.grad for p in params], accumulate, mask_sum, global_rays, density_normal)
+    return params
 
 
 class _FusedLoss(torch.autograd.Function):
